@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — counter-samples/sec of the telemetry hot path (BASELINE.json metric) on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (config.workload, BASELINE configs[3] per GPU): 512 fields x 1 Mi-sample f64 ring (4 GiB, >> the 126 MB L2, so
@@ -21,6 +21,9 @@ on a side stream (the exchange has no data dependency on the reduce).  Weak scal
            a slower selection path), `range` is the whole-ring (W = CAP) order statistic of configs[3].
 `verify`   the WHOLE 512 x 1 Mi result of the last timed step against the C oracle (bit-exact selections and counts, max relative
            error of mean / EMA), and the W = CAP result the same way.
+`--dump-outputs DIR`  the six [512][1049] aggregates of the last timed step (rank 0's ring) as DIR/<op>.npy, float64 (n_over
+           widened exactly), 26 MB in all.  The stream is seeded, so two builds run with the same arguments can be compared
+           output for output.
 `cpu_baseline` / `--impl reference`: the C oracle (oracle/oracle.c, kind "port": the Go reference cannot be built here and has no
            windowed aggregation at all) rebuilt -O3 -march=native on this host, on the CPUs this process may really use
            (affinity and cgroup quota, not `nproc`), bounded sample, rank 0 only.
@@ -146,6 +149,13 @@ def cpu_leg(steps, warmup, fields, ring=None, thr=None):
             "achieved_GBps": v * 8 / 1e9, "build": note, "host_cpus": cpus}, dt
 
 
+def dump_outputs(d, got):
+    """what a caller of the reduce receives, one .npy per aggregate; float64 holds every uint32 n_over exactly"""
+    os.makedirs(d, exist_ok=True)
+    for k, v in got.items():
+        np.save(os.path.join(d, k + ".npy"), v.astype(np.float64))
+
+
 def verify_windows(got, ring_host, thr, coracle):
     """the whole [F][nw] result against the C oracle on the same samples: exact selections / counts, max relative error of the float ones"""
     want = coracle.windows_fields(ring_host, W, thr)
@@ -196,6 +206,7 @@ def main():
     ap.add_argument("--no-scan", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-shapes", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the aggregates of the last timed step to DIR/<op>.npy")
     a = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -208,6 +219,8 @@ def main():
               "l2": "input 4 GiB per GPU >> 126 MB L2; every step re-streams HBM"}
 
     if a.impl == "reference":
+        if a.dump_outputs:
+            ap.error("--dump-outputs writes the device result: --impl b200 only")
         # The reference's own CPU path for this metric does not exist (no windowed aggregation in gpud) and Go cannot be
         # built here; the timed arm is the C oracle port with every CPU this process may use.  Rank 0 only.
         if rank != 0:
@@ -338,7 +351,10 @@ def main():
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
     # the result of the last timed step, before anything else touches the ring
-    got = {k: ring.read(k) for k in g.OPS} if do_verify else None
+    do_dump = rank == 0 and a.dump_outputs
+    got = {k: ring.read(k) for k in g.OPS} if do_verify or do_dump else None
+    if do_dump:
+        dump_outputs(a.dump_outputs, got)
     # per-kernel device time of the dominant kernel: the same step K more times, reading the library's own events
     kms = []
     for _ in range(a.steps):

@@ -1203,6 +1203,17 @@ def test_poller_gpm_metrics_against_nvml(ctx):
         m = poller.gpm_metrics(50)
         assert m.supported == 0 and g.capi.gpm_check([m]) == (0, "GPM not supported")
         return
+    s0 = pynvml.nvmlGpmSampleAlloc()
+    try:                                             # some hosts report GPM support and then refuse every sample (NVML_ERROR_UNKNOWN)
+        pynvml.nvmlGpmSampleGet(h, s0)
+    except pynvml.NVMLError as e:
+        import re
+        for call in (lambda: poller.gpm_metrics(10), lambda: poller.poll_gpm(ring, 1, 10)):
+            with pytest.raises(g.GpudError, match=re.escape(str(e))):   # NVML's refusal is passed on, no reading is made up
+                call()
+        pytest.skip("NVML reports GPM support but refuses GPM samples on this host: %s" % e)
+    finally:
+        pynvml.nvmlGpmSampleFree(s0)
     stop = threading.Event()
 
     def load():

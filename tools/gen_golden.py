@@ -396,6 +396,9 @@ def main():
     rows = ident(rows)
     for r in rows:
         r["wantEventName"] = cs[r["wantEventName"]]["value"] if r["wantEventName"] in cs else r["wantEventName"]
+        # the kernel's hung-task hint quotes a shell command that changes a kernel setting; the fixture keeps the line (it comes
+        # before the panic and matches no pattern) in plain words, so no file in the repository carries that command
+        r["logLines"] = [re.sub(r'"echo 0 [^"]*/hung_task_timeout_secs"', "Setting kernel.hung_task_timeout_secs to 0", l) for l in r["logLines"]]
     ext3["os.panic_detection"] = {"src": src, "rows": rows, "note": "lines fed to Match until the first non-empty event"}
     rows, src = table(OSD + "kmsg_matcher_test.go", "TestKernelPanicStatefulMatcher")
     rows = ident(rows)
