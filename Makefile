@@ -8,7 +8,7 @@ LIB := gpud_b200/libgpud_b200.so
 
 all: $(LIB) gpud_b200/gpud-scan oracle
 
-$(SRC)/%.o: $(SRC)/%.cu $(SRC)/internal.h $(SRC)/catalog.h include/gpud_b200.h
+$(SRC)/%.o: $(SRC)/%.cu $(SRC)/internal.h $(SRC)/catalog.h $(SRC)/ring_drain.h include/gpud_b200.h
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $@.ptxas.log || (cat $@.ptxas.log; exit 1)
 
 $(SRC)/catalog.o: $(SRC)/catalog.cpp $(SRC)/catalog.h $(SRC)/catalog_data.inc include/gpud_b200.h
@@ -17,13 +17,13 @@ $(SRC)/catalog.o: $(SRC)/catalog.cpp $(SRC)/catalog.h $(SRC)/catalog_data.inc in
 $(SRC)/host_component.o: $(SRC)/host_component.cpp $(SRC)/host_component.h $(SRC)/json_min.h include/gpud_b200.h
 	g++ -O2 -std=c++17 -fPIC -Wall -c $< -o $@
 
-$(SRC)/component_abi.o: $(SRC)/component_abi.cpp $(SRC)/host_component.h $(SRC)/internal.h include/gpud_b200.h
+$(SRC)/component_abi.o: $(SRC)/component_abi.cpp $(SRC)/host_component.h $(SRC)/internal.h $(SRC)/ring_drain.h include/gpud_b200.h
 	g++ -O2 -std=c++17 -fPIC -Wall -I/usr/local/cuda/include -c $< -o $@
 
 $(SRC)/poller.o: $(SRC)/poller.cpp $(SRC)/internal.h include/gpud_b200.h
 	g++ -O2 -std=c++17 -fPIC -Wall -I/usr/local/cuda/include -c $< -o $@
 
-$(SRC)/store_sqlite.o: $(SRC)/store_sqlite.cpp $(SRC)/json_min.h include/gpud_b200.h
+$(SRC)/store_sqlite.o: $(SRC)/store_sqlite.cpp $(SRC)/json_min.h $(SRC)/ring_drain.h include/gpud_b200.h
 	g++ -O2 -std=c++17 -fPIC -Wall -c $< -o $@
 
 $(SRC)/kmsg_stateful.o: $(SRC)/kmsg_stateful.cpp include/gpud_b200.h

@@ -5,7 +5,7 @@ binding over that C ABI used by the tests and bench.py; it contains no compute a
 point raises if the shared library or a CUDA device is missing.
 """
 from .capi import (Context, GpudError, Ring, FabricRaw, FabricLocal, FabricVerdict, XidHit, lib, OPS, EVENT_NAMES,
-                   ACTION_WIRE, SCAN_LINES, SCAN_RAW_KMSG, SCAN_EXT_MATCHERS, DTYPES, KmsgStateful, KmsgEvent, Poller, POLL_FIELDS, IbSnapshot, IbVerdict, ib_reason, Store, Metric, DedupRule, EventRow, xid_build_message, xid_hit_message, xid_detail, Temperature, PollCounters, temperature_check, fabric_reason, hw_slowdown_event_message, hw_slowdown_check, temperature_reason, fabric_report_reason)
+                   ACTION_WIRE, SCAN_LINES, SCAN_RAW_KMSG, SCAN_EXT_MATCHERS, DTYPES, KmsgStateful, KmsgEvent, Poller, POLL_FIELDS, IbSnapshot, IbVerdict, ib_reason, Store, Metric, DedupRule, EventRow, xid_build_message, xid_hit_message, xid_detail, Temperature, PollCounters, temperature_check, fabric_reason, hw_slowdown_event_message, hw_slowdown_check, temperature_reason, fabric_report_reason, DrainInfo, window_metric_name)
 
 __all__ = ["Context", "GpudError", "Ring", "FabricRaw", "FabricLocal", "FabricVerdict", "XidHit", "lib", "OPS",
-           "EVENT_NAMES", "ACTION_WIRE", "SCAN_LINES", "SCAN_RAW_KMSG", "SCAN_EXT_MATCHERS", "DTYPES", "KmsgStateful", "KmsgEvent", "Poller", "POLL_FIELDS", "IbSnapshot", "IbVerdict", "ib_reason", "Store", "Metric", "DedupRule", "EventRow", "xid_build_message", "xid_hit_message", "xid_detail", "Temperature", "PollCounters", "temperature_check", "fabric_reason", "hw_slowdown_event_message", "hw_slowdown_check", "temperature_reason", "fabric_report_reason"]
+           "EVENT_NAMES", "ACTION_WIRE", "SCAN_LINES", "SCAN_RAW_KMSG", "SCAN_EXT_MATCHERS", "DTYPES", "KmsgStateful", "KmsgEvent", "Poller", "POLL_FIELDS", "IbSnapshot", "IbVerdict", "ib_reason", "Store", "Metric", "DedupRule", "EventRow", "xid_build_message", "xid_hit_message", "xid_detail", "Temperature", "PollCounters", "temperature_check", "fabric_reason", "hw_slowdown_event_message", "hw_slowdown_check", "temperature_reason", "fabric_report_reason", "DrainInfo", "window_metric_name"]

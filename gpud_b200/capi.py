@@ -57,6 +57,22 @@ class Metric(C.Structure):
     _fields_ = [("unix_ms", C.c_int64), ("component", C.c_char_p), ("name", C.c_char_p), ("labels_json", C.c_char_p), ("value", C.c_double)]
 
 
+class DrainInfo(C.Structure):
+    _fields_ = [("first_window", C.c_int64), ("n_windows", C.c_int64), ("n_lost", C.c_int64), ("n_pending", C.c_int64)]
+
+    def as_dict(self) -> dict:
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
+
+
+def window_metric_name(field: str, op: str, q_num: int = 99, q_den: int = 100) -> str:
+    """gpud_window_metric_name: "<field>_window_<op>" (op one of OPS; the order statistic is named p<Q>)"""
+    out = C.create_string_buffer(512)
+    n = lib().gpud_window_metric_name(field.encode(), OPS[op], q_num, q_den, out, 512)
+    if n < 0:
+        raise GpudError(n, "gpud_window_metric_name")
+    return out.value.decode()
+
+
 def hw_slowdown_event_message(bitmask: int, gpu_uuid: str) -> str:
     buf = C.create_string_buffer(2048)
     n = lib().gpud_hw_slowdown_event_message(bitmask, gpu_uuid.encode(), buf, 2048)
@@ -246,6 +262,12 @@ class Store:
         arr = (XidHit * max(1, len(hits)))(*hits)
         n = C.c_int32()
         self._check(self._L.gpud_kmsg_syncer_feed(sy, kmsg_component.encode(), arr, len(hits), C.cast(C.c_char_p(buf), C.c_void_p), boot_unix, now_unix, C.byref(n)))
+        return n.value
+
+    def purge_metrics(self, before_unix_ms: int, table: str = "") -> int:
+        """purge (metrics/store/sqlite.go:258-275): deletes the rows older than before_unix_ms; returns how many"""
+        n = C.c_int64()
+        self._check(self._L.gpud_store_purge_metrics(self._h, table.encode(), before_unix_ms, C.byref(n)))
         return n.value
 
     def metrics_table(self, table: str = ""):
@@ -615,6 +637,11 @@ class Component:
     def ring_handle(self, slot: int = 0):
         return self._L.gpud_component_ring(self._h, slot)
 
+    def set_metrics_store(self, store: Optional["Store"], table: str = ""):
+        """temperature only: drain every GPU's ring into `store` on each Check (None detaches)"""
+        self.ctx._check(self._L.gpud_component_set_metrics_store(self._h, store._h if store is not None else None, table.encode()))
+        self._store = store                    # the store must outlive the attachment
+
     def close(self):
         if self._h:
             self._L.gpud_component_close(self._h)
@@ -681,8 +708,9 @@ class FabricVerdict(C.Structure):
 SYMBOLS = ["gpud_abi_version", "gpud_sizeof", "gpud_ctx_create", "gpud_ctx_destroy", "gpud_last_error", "gpud_host_alloc",
            "gpud_host_free", "gpud_ring_create", "gpud_ring_destroy", "gpud_ring_set_stream", "gpud_ring_push",
            "gpud_ring_push_device", "gpud_ring_push_raw", "gpud_clock_event_reasons", "gpud_hw_slowdown_event_message", "gpud_hw_slowdown_check", "gpud_store_insert_hw_slowdown", "gpud_store_open", "gpud_store_close", "gpud_store_last_error", "gpud_store_event_table", "gpud_store_insert_event", "gpud_store_insert_xid_hits", "gpud_store_metrics_table", "gpud_store_record_metrics", "gpud_kmsg_syncer_create", "gpud_kmsg_syncer_destroy", "gpud_kmsg_syncer_feed", "gpud_store_find_event", "gpud_store_record_reboot", "gpud_xid_state_from_store", "gpud_sxid_state_from_store", "gpud_store_get_events", "gpud_store_latest_event", "gpud_store_purge_events", "gpud_kmsg_syncer_configure", "gpud_kmsg_syncer_configure_component", "gpud_kmsg_syncer_offer", "gpud_ib_scan", "gpud_ib_reason", "gpud_poller_create", "gpud_poller_destroy", "gpud_poller_poll", "gpud_poller_last_rows", "gpud_poller_errors", "gpud_poll_row_hold", "gpud_nvml_devices", "gpud_nvml_devices_arg", "gpud_nvml_bus_id", "gpud_poller_remapped_rows", "gpud_remapped_rows_check", "gpud_poller_ecc_errors", "gpud_poller_field_row", "gpud_poller_poll_fields", "gpud_poller_gpm_supported", "gpud_poller_gpm_metrics", "gpud_poller_poll_gpm", "gpud_gpm_check", "gpud_poller_fabric_raw", "gpud_poller_product_name", "gpud_poller_temperature", "gpud_temperature_check", "gpud_temperature_reason", "gpud_poller_counters", "gpud_ring_counts", "gpud_ring_reduce", "gpud_ring_sync", "gpud_ring_kernel_ms", "gpud_ring_read",
-           "gpud_ring_result_ptr", "gpud_ring_reduce_range", "gpud_ring_range_stats", "gpud_ring_set_cta_reserve", "gpud_kmsg_scan", "gpud_kmsg_scan_sharded", "gpud_kmsg_scan_device", "gpud_kmsg_scan_kernel_ms", "gpud_kmsg_scan_phase_timing", "gpud_kmsg_scan_stats", "gpud_xid_classify",
-           "gpud_hit_detail_json", "gpud_xid_description", "gpud_xid_mnemonic", "gpud_sxid_name", "gpud_nvlink_rule_hint", "gpud_sxid_reason", "gpud_sxid_get_detail", "gpud_store_insert_sxid_hits", "gpud_product_mem_caps", "gpud_product_fm_supported", "gpud_product_fabric_state_supported", "gpud_xid_get_detail", "gpud_xid_detail", "gpud_xid_build_message", "gpud_xid_hit_message", "gpud_xid_device_matches_bus_id", "gpud_kmsg_event_name", "gpud_kmsg_event_message", "gpud_kmsg_component", "gpud_kmsg_hit_message", "gpud_kmsg_stateful_create", "gpud_kmsg_stateful_destroy", "gpud_kmsg_stateful_feed", "gpud_component_create", "gpud_component_destroy", "gpud_component_name", "gpud_component_start", "gpud_component_check", "gpud_component_last_health_states", "gpud_component_events", "gpud_component_close", "gpud_component_checks", "gpud_component_xid_set_source", "gpud_component_xid_set_healthy", "gpud_component_xid_add_reboot", "gpud_component_xid_set_devices", "gpud_component_ring", "gpud_kmsg_stateful_feed_units", "gpud_kmsg_deduper_create", "gpud_kmsg_deduper_destroy", "gpud_kmsg_dedup_units",
+           "gpud_ring_result_ptr", "gpud_ring_reduce_range", "gpud_ring_range_stats", "gpud_ring_drain", "gpud_ring_push_timed", "gpud_ring_drain_to_store",
+           "gpud_store_purge_metrics", "gpud_window_metric_name", "gpud_ring_set_cta_reserve", "gpud_kmsg_scan", "gpud_kmsg_scan_sharded", "gpud_kmsg_scan_device", "gpud_kmsg_scan_kernel_ms", "gpud_kmsg_scan_phase_timing", "gpud_kmsg_scan_stats", "gpud_xid_classify",
+           "gpud_hit_detail_json", "gpud_xid_description", "gpud_xid_mnemonic", "gpud_sxid_name", "gpud_nvlink_rule_hint", "gpud_sxid_reason", "gpud_sxid_get_detail", "gpud_store_insert_sxid_hits", "gpud_product_mem_caps", "gpud_product_fm_supported", "gpud_product_fabric_state_supported", "gpud_xid_get_detail", "gpud_xid_detail", "gpud_xid_build_message", "gpud_xid_hit_message", "gpud_xid_device_matches_bus_id", "gpud_kmsg_event_name", "gpud_kmsg_event_message", "gpud_kmsg_component", "gpud_kmsg_hit_message", "gpud_kmsg_stateful_create", "gpud_kmsg_stateful_destroy", "gpud_kmsg_stateful_feed", "gpud_component_create", "gpud_component_destroy", "gpud_component_name", "gpud_component_start", "gpud_component_check", "gpud_component_last_health_states", "gpud_component_events", "gpud_component_close", "gpud_component_checks", "gpud_component_xid_set_source", "gpud_component_xid_set_healthy", "gpud_component_xid_add_reboot", "gpud_component_xid_set_devices", "gpud_component_ring", "gpud_component_set_metrics_store", "gpud_kmsg_stateful_feed_units", "gpud_kmsg_deduper_create", "gpud_kmsg_deduper_destroy", "gpud_kmsg_dedup_units",
            "gpud_fabric_issues", "gpud_fabric_suggest_reboot", "gpud_set_nvml_error_string", "gpud_nvml_error_strings_from_driver", "gpud_fabric_reason", "gpud_fabric_report_reason", "gpud_fabric_pack", "gpud_fabric_verdict_device", "gpud_comm_unique_id", "gpud_comm_init", "gpud_fabric_gather",
            "gpud_fabric_gather_p2p"]
 
@@ -738,6 +766,10 @@ def lib() -> C.CDLL:
         "gpud_ring_kernel_ms": (i32, [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]), "gpud_ring_read": (i32, [vp, i32, vp, i64]),
         "gpud_ring_result_ptr": (i32, [vp, i32, C.POINTER(vp)]), "gpud_ring_reduce_range": (i32, [vp, i64, vp, vp]),
         "gpud_ring_set_cta_reserve": (i32, [vp, i32]),
+        "gpud_ring_drain": (i32, [vp, i64, vp, vp, vp, C.POINTER(DrainInfo)]), "gpud_ring_push_timed": (i32, [vp, vp, i64, i32, vp]),
+        "gpud_ring_drain_to_store": (i32, [vp, vp, C.c_char_p, vp, vp, C.c_char_p, C.c_uint32, i64, C.POINTER(DrainInfo), C.POINTER(i64), C.POINTER(i64)]),
+        "gpud_store_purge_metrics": (i32, [vp, C.c_char_p, i64, C.POINTER(i64)]), "gpud_window_metric_name": (i32, [C.c_char_p, i32, i32, i32, vp, i32]),
+        "gpud_component_set_metrics_store": (i32, [vp, vp, C.c_char_p]),
         "gpud_ring_range_stats": (i32, [vp, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_int32), vp]),
         "gpud_kmsg_scan": (i32, [vp, i32, vp, i64, i32, C.POINTER(XidHit), i64, C.POINTER(i64), C.POINTER(i64)]),
         "gpud_kmsg_scan_sharded": (i32, [vp, vp, i64, i32, C.POINTER(XidHit), i64, C.POINTER(i64), C.POINTER(i64)]),
@@ -779,7 +811,7 @@ def lib() -> C.CDLL:
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
         fn.restype, fn.argtypes = res, args
-    for which, st in enumerate((XidHit, FabricRaw, FabricLocal, FabricVerdict, RingCfg, KmsgEvent, IbSnapshot, IbVerdict, Metric, DedupRule, Temperature, PollCounters, EventRow, NvmlDevice, RemappedRows, EccErrors, GpmMetrics)):
+    for which, st in enumerate((XidHit, FabricRaw, FabricLocal, FabricVerdict, RingCfg, KmsgEvent, IbSnapshot, IbVerdict, Metric, DedupRule, Temperature, PollCounters, EventRow, NvmlDevice, RemappedRows, EccErrors, GpmMetrics, DrainInfo)):
         if L.gpud_sizeof(which) != C.sizeof(st):
             raise GpudError(-1, "ABI layout mismatch for %s: C %d vs ctypes %d" % (st.__name__, L.gpud_sizeof(which), C.sizeof(st)))
     _lib = L
@@ -1034,6 +1066,50 @@ class Ring:
     def reduce_all(self) -> dict:
         self.reduce()
         return {k: self.read(k) for k in OPS}
+
+    def push_timed(self, rows: np.ndarray, unix_ms):
+        """push_raw with the unix-ms time of every row (non-decreasing, not before the last timed row)"""
+        rows = np.ascontiguousarray(rows)
+        assert rows.ndim == 2 and rows.shape[1] == self.F
+        ms = np.ascontiguousarray(unix_ms, dtype=np.int64)
+        assert ms.shape == (rows.shape[0],)
+        self.ctx._check(self._L.gpud_ring_push_timed(self._h, C.c_void_p(rows.ctypes.data), rows.shape[0], DTYPES[rows.dtype.name],
+                                                     C.c_void_p(ms.ctypes.data)))
+
+    def drain(self, max_windows: int) -> dict:
+        """gpud_ring_drain: the next complete stream-aligned windows, each [F][n] like reduce_all, plus "window_end_unix_ms" [n] and
+        "info" {first_window, n_windows, n_lost, n_pending}.  max_windows = 0 only reports the counts."""
+        mw = max(0, int(max_windows))
+        f64 = np.empty((5, self.F, max(1, mw)), dtype=np.float64)
+        nov = np.empty((self.F, max(1, mw)), dtype=np.uint32)
+        ms = np.empty((max(1, mw),), dtype=np.int64)
+        info = DrainInfo()
+        self.ctx._check(self._L.gpud_ring_drain(self._h, mw, C.c_void_p(f64.ctypes.data), C.c_void_p(nov.ctypes.data), C.c_void_p(ms.ctypes.data),
+                                                C.byref(info)))
+        n = info.n_windows
+        out = {k: f64[OPS[k]][:, :n].copy() for k in ("min", "max", "mean", "ema", "p99")}
+        out["n_over"] = nov[:, :n].copy()
+        out["window_end_unix_ms"] = ms[:n].copy()
+        out["info"] = info.as_dict()
+        return out
+
+    def drain_to_store(self, store: "Store", components, field_names, labels_json: str = "", ops_mask: int = 0, max_windows: int = 1 << 20,
+                       table: str = ""):
+        """gpud_ring_drain_to_store: one metrics row per returned window x named field x op; field_names[f] None skips field f.
+        Returns (info dict, rows written, windows moved to keep their times increasing)."""
+        assert len(components) == self.F and len(field_names) == self.F
+        comps = [c.encode() if c is not None else None for c in components]
+        names = [f.encode() if f is not None else None for f in field_names]
+        ca, na = (C.c_char_p * self.F)(*comps), (C.c_char_p * self.F)(*names)
+        info, rows, shifted = DrainInfo(), C.c_int64(), C.c_int64()
+        rc = self._L.gpud_ring_drain_to_store(self._h, store._h, table.encode(), ca, na, labels_json.encode(), ops_mask, max_windows, C.byref(info),
+                                              C.byref(rows), C.byref(shifted))
+        if rc:
+            sb, cb = C.create_string_buffer(512), C.create_string_buffer(512)
+            self._L.gpud_store_last_error(store._h, sb, 512)
+            self._L.gpud_last_error(self.ctx._h, cb, 512)
+            raise GpudError(rc, "%s (ring: %s)" % (sb.value.decode("utf-8", "replace"), cb.value.decode("utf-8", "replace")))
+        return info.as_dict(), rows.value, shifted.value
 
     def reduce_range(self, last_n: int = 0) -> dict:
         f64 = np.empty((5, self.F), dtype=np.float64)

@@ -73,7 +73,7 @@ extern "C" int32_t gpud_host_free(void* p) {
 }
 
 // struct sizes for binding layout checks (ctypes / cgo): 0 hit, 1 fabric_raw, 2 fabric_local, 3 fabric_verdict, 4 ring_cfg,
-// 5 kmsg_event, 6 ib_snapshot, 7 ib_verdict, 8 metric, 9 dedup_rule, 10 temperature, 11 poll_counters, 12 event_row
+// 5 kmsg_event, 6 ib_snapshot, 7 ib_verdict, 8 metric, 9 dedup_rule, 10 temperature, 11 poll_counters, 12 event_row, .., 17 drain_info
 extern "C" int32_t gpud_sizeof(int32_t which) {
   switch (which) {
     case 0: return (int32_t)sizeof(gpud_xid_hit);
@@ -93,6 +93,7 @@ extern "C" int32_t gpud_sizeof(int32_t which) {
     case 14: return (int32_t)sizeof(gpud_remapped_rows);
     case 15: return (int32_t)sizeof(gpud_ecc_errors);
     case 16: return (int32_t)sizeof(gpud_gpm_metrics);
+    case 17: return (int32_t)sizeof(gpud_drain_info);
   }
   return -1;
 }

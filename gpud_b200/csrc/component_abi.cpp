@@ -16,6 +16,7 @@
 
 #include "host_component.h"
 #include "internal.h"
+#include "ring_drain.h"
 
 namespace {
 
@@ -52,8 +53,20 @@ void close_slots(std::vector<DevSlot>* slots) {
   slots->clear();
 }
 
+// The poll columns as the reference's gauges name them: component_name = the component that owns the gauge, metric name = SubSystem +
+// gauge name (components/accelerator/nvidia/{temperature,power,clock-speed,utilization,memory}/metrics.go).  The reference has no SM
+// clock gauge, and its memory gauge counts bytes where this column counts MiB: those two names say what the column holds.
+const char* const kPollComponent[GPUD_POLL_N_FIELDS] = {
+    "accelerator-nvidia-temperature", "accelerator-nvidia-power", "accelerator-nvidia-clock-speed", "accelerator-nvidia-clock-speed",
+    "accelerator-nvidia-clock-speed", "accelerator-nvidia-utilization", "accelerator-nvidia-utilization", "accelerator-nvidia-memory"};
+const char* const kPollMetric[GPUD_POLL_N_FIELDS] = {
+    "accelerator_nvidia_temperature_current_celsius", "accelerator_nvidia_power_current_usage_milli_watts",
+    "accelerator_nvidia_clock_speed_graphics_mhz", "accelerator_nvidia_clock_speed_sm_mhz", "accelerator_nvidia_clock_speed_memory_mhz",
+    "accelerator_nvidia_utilization_gpu_util_percent", "accelerator_nvidia_utilization_memory_util_percent", "accelerator_nvidia_memory_used_mib"};
+
 // temperature: one poll row per check into the ring (the windowed aggregates stay available through gpud_component_ring), the
-// reference's rules over the current reading (temperature/component.go:190-287)
+// reference's rules over the current reading (temperature/component.go:190-287); with a metrics store attached, every completed window
+// of the ring goes into the store right after the poll (the Syncer's job in the reference, pkg/metrics/syncer/syncer.go:36-82)
 class TemperatureComponent : public gpud::Component {
  public:
   static constexpr const char* kName = "accelerator-nvidia-temperature";            // temperature/component.go:27
@@ -73,6 +86,7 @@ class TemperatureComponent : public gpud::Component {
     std::vector<const char*> uuids;
     for (size_t i = 0; i < slots_.size(); ++i) {
       int32_t rc = gpud_poller_poll(slots_[i].poller, 1, 0);                          // the sample sink: one row into the ring
+      if (rc == GPUD_OK && store_) sync_metrics(slots_[i]);
       if (rc == GPUD_OK) rc = gpud_poller_temperature(slots_[i].poller, &ts[i]);
       if (rc != GPUD_OK) {                                                            // "error getting temperature" (:196-204)
         char msg[512] = {0};
@@ -101,7 +115,34 @@ class TemperatureComponent : public gpud::Component {
   std::vector<gpud::Event> Events(int64_t) override { return {}; }                    // temperature/component.go:118-120: no events
   int32_t Close() override { return 0; }
   gpud_ring* ring(int slot) { return slot >= 0 && slot < (int)slots_.size() ? slots_[slot].ring : nullptr; }
+  // caller holds the component's check lock
+  int32_t SetMetricsStore(gpud_store* st, const char* table) {
+    if (st) {
+      const int32_t rc = gpud_store_metrics_table(st, table);                         // CreateTable (metrics/store/sqlite.go:87-106)
+      if (rc != GPUD_OK) return rc;
+    }
+    store_ = st;
+    table_ = table ? table : "";
+    return GPUD_OK;
+  }
  private:
+  // A failed drain leaves the check result alone (the reference Syncer only logs, syncer.go:52-54) and the windows where they are
+  void sync_metrics(const DevSlot& s) {
+    std::string labels = "{\"uuid\":";
+    gpud::jstr(labels, s.uuid);
+    labels += "}";
+    gpud_drain_info info;
+    const int32_t rc = gpud_ring_drain_to_store(s.ring, store_, table_.c_str(), kPollComponent, kPollMetric, labels.c_str(), 0, kMaxDrain, &info,
+                                                nullptr, nullptr);
+    if (rc != GPUD_OK) {
+      char msg[512] = {0};
+      gpud_store_last_error(store_, msg, sizeof msg);
+      gpud_fail(ctx_, rc, "metrics drain of %s: %s", s.uuid.c_str(), msg);
+    }
+  }
+  static constexpr int64_t kMaxDrain = 128;                                            // > the 66 windows a 64 Ki-sample ring holds
+  gpud_store* store_ = nullptr;
+  std::string table_;
   void store(const HealthState& s) { std::lock_guard<std::mutex> g(mu_); last_ = s; checked_ = true; }
   gpud_ctx* ctx_;
   int32_t margin_;
@@ -342,3 +383,8 @@ extern "C" int32_t gpud_component_xid_set_devices(gpud_component* c, const char*
 }
 // temperature only: the ring the component's polls land in (device slot of the ctx), for gpud_ring_reduce / gpud_ring_read
 extern "C" gpud_ring* gpud_component_ring(gpud_component* c, int32_t slot) { return (c && c->temp) ? c->temp->ring(slot) : nullptr; }
+extern "C" int32_t gpud_component_set_metrics_store(gpud_component* c, gpud_store* st, const char* table) {
+  if (!c || !c->temp) return GPUD_E_INVALID;
+  std::lock_guard<std::mutex> g(c->check_mu);
+  return c->temp->SetMetricsStore(st, table);
+}

@@ -1,5 +1,6 @@
 // poller.cpp — real ingest (SURVEY.md 8f.3): the host poller that reads the NVML gauges of one GPU and feeds K1 with raw
-// uint32 poll rows through pinned memory (gpud_ring_push_raw).  The getters are the ones the reference's components call
+// uint32 poll rows through pinned memory (gpud_ring_push_timed: every row carries the wall-clock ms its getters returned at, which
+// the streaming drain turns into the end time of each window).  The getters are the ones the reference's components call
 // once per minute and widen with metric.Set(float64(v)):
 //   temperature C     dev.GetTemperature(nvml.TEMPERATURE_GPU)        components/accelerator/nvidia/temperature/temperature.go:85
 //   power mW          dev.GetPowerUsage()                              components/accelerator/nvidia/power/power.go:46
@@ -128,7 +129,18 @@ struct gpud_poller {
   uint64_t* field_rows = nullptr;                // pinned [cap_rows][GPUD_FIELD_ROW_N] (gpud_poller_poll_fields)
   uint64_t field_held[GPUD_FIELD_ROW_N] = {0};
   double gpm_held[GPUD_GPM_N] = {0};
+  std::vector<int64_t> row_ms;                   // [cap_rows]: unix ms of each row of the batch being polled
+  int64_t last_ms = INT64_MIN;                   // the newest row time handed out (row times never go back, even if the clock does)
 };
+
+// CLOCK_REALTIME in ms, taken as soon as a row's getters have returned; clamped so that a clock step back cannot make a row older
+// than the one before it (gpud_ring_push_timed refuses that)
+static int64_t row_time_ms(gpud_poller* p) {
+  timespec ts;
+  clock_gettime(CLOCK_REALTIME, &ts);
+  p->last_ms = std::max(p->last_ms, (int64_t)ts.tv_sec * 1000 + ts.tv_nsec / 1000000);
+  return p->last_ms;
+}
 
 extern "C" int32_t gpud_poller_create(gpud_ctx* ctx, int32_t dev, gpud_ring* ring, gpud_poller** out) {
   if (!ctx || !ring || !out) return GPUD_E_INVALID;
@@ -143,6 +155,7 @@ extern "C" int32_t gpud_poller_create(gpud_ctx* ctx, int32_t dev, gpud_ring* rin
   gpud_poller* p = new gpud_poller();
   p->ctx = ctx; p->ring = ring; p->dev = dev; p->h = h;
   p->cap_rows = 1 << 14;
+  p->row_ms.assign((size_t)p->cap_rows, 0);
   if (cudaMallocHost(&p->rows, (size_t)p->cap_rows * GPUD_POLL_N_FIELDS * sizeof(uint32_t)) != cudaSuccess) {
     delete p;
     return gpud_fail(ctx, GPUD_E_CUDA, "pinned poll buffer");
@@ -217,10 +230,11 @@ extern "C" int32_t gpud_poller_poll(gpud_poller* p, int64_t n_polls, int64_t int
     const int64_t batch = std::min<int64_t>(p->cap_rows, n_polls - done);
     for (int64_t i = 0; i < batch; ++i) {
       poll_row(N, p, p->rows + i * GPUD_POLL_N_FIELDS);
+      p->row_ms[i] = row_time_ms(p);
       if (interval_us) { timespec ts{(time_t)(interval_us / 1000000), (long)(interval_us % 1000000) * 1000L}; nanosleep(&ts, nullptr); }
     }
     p->n_rows = batch;
-    const int32_t rc = gpud_ring_push_raw(p->ring, p->rows, batch, GPUD_DT_U32);   // pinned: direct DMA + widening append, synchronous return
+    const int32_t rc = gpud_ring_push_timed(p->ring, p->rows, batch, GPUD_DT_U32, p->row_ms.data());   // pinned: direct DMA + widening append, synchronous return
     if (rc) return rc;
     done += batch;
   }
@@ -643,6 +657,7 @@ extern "C" int32_t gpud_poller_poll_fields(gpud_poller* p, gpud_ring* ring, int6
       uint64_t v[GPUD_FIELD_ROW_N];
       int32_t rcs[GPUD_FIELD_ROW_N];
       const int32_t rc = field_row(N, p->h, v, rcs);
+      p->row_ms[i] = row_time_ms(p);
       uint64_t* row = p->field_rows + i * GPUD_FIELD_ROW_N;
       for (int c = 0; c < GPUD_FIELD_ROW_N; ++c) {
         if (rc == 0 && rcs[c] == 0) p->field_held[c] = v[c];
@@ -650,7 +665,7 @@ extern "C" int32_t gpud_poller_poll_fields(gpud_poller* p, gpud_ring* ring, int6
       }
       if (interval_us) { timespec ts{(time_t)(interval_us / 1000000), (long)(interval_us % 1000000) * 1000L}; nanosleep(&ts, nullptr); }
     }
-    const int32_t rc = gpud_ring_push_raw(ring, p->field_rows, batch, GPUD_DT_U64);
+    const int32_t rc = gpud_ring_push_timed(ring, p->field_rows, batch, GPUD_DT_U64, p->row_ms.data());
     if (rc) return rc;
     done += batch;
   }
@@ -773,12 +788,13 @@ extern "C" int32_t gpud_poller_poll_gpm(gpud_poller* p, gpud_ring* ring, int64_t
     gpud_gpm_metrics m;
     r = gpm_between(p, N, prev, next, &m);
     if (r) return r;
+    const int64_t ms = row_time_ms(p);
     double row[GPUD_GPM_N];
     for (int c = 0; c < GPUD_GPM_N; ++c) {                                  // a metric NVML could not compute holds its last good value
       if (m.nvml_rc[c] == 0) p->gpm_held[c] = m.value[c];
       row[c] = p->gpm_held[c];
     }
-    r = gpud_ring_push(ring, row, 1);
+    r = gpud_ring_push_timed(ring, row, 1, GPUD_DT_F64, &ms);
     if (r) return r;
     std::swap(prev, next);
   }

@@ -19,6 +19,7 @@
 #include <algorithm>
 
 #include "internal.h"
+#include "ring_drain.h"
 
 namespace {
 
@@ -958,10 +959,13 @@ __global__ void __launch_bounds__(kIpWarps * 32, 1) k_window_reduce_inplace(cons
 // K3 carry: E_w = (1-alpha)^{m_w} E_{w-1} + P_w, E_{-1} = x[0] (oldest sample).  One 128-thread CTA per field:
 // rows of 128 consecutive windows are scanned with a decayed Kogge-Stone prefix (S_t += d^off S_{t-off}), the carry
 // crosses rows through shared memory; only the last window can have a different decay.
+// SEEDED (the streaming drain): E_{-1} = seed_in[f], the EMA the previous drain ended on, instead of the first sample.  When seed_out
+// is set, E of the last window is written there (seed_in may alias it: one thread reads it first and writes it last).
 // ---------------------------------------------------------------------------------------------
+template <bool SEEDED>
 __global__ void __launch_bounds__(128) k_ema_carry(const double* __restrict__ part, const double* __restrict__ ring, int64_t cap,
                                                     int64_t start, int F, int nw, double d_full, double d_last,
-                                                    double* __restrict__ out_ema) {
+                                                    double* __restrict__ out_ema, const double* seed_in, double* seed_out) {
   __shared__ double s_warp[4];
   __shared__ double s_carry;
   const int f = blockIdx.x, t = threadIdx.x, lane = t & 31, wid = t >> 5;
@@ -973,7 +977,7 @@ __global__ void __launch_bounds__(128) k_ema_carry(const double* __restrict__ pa
   for (int i = 1; i < 6; ++i) dp[i] = dp[i - 1] * dp[i - 1];
   const double my_pow = pow(d_full, (double)(t + 1));        // d^(t+1): weight of the incoming carry at position t of a row
   const double lane_pow = pow(d_full, (double)(lane + 1));
-  if (t == 0) s_carry = ring[(int64_t)f * cap + start];
+  if (t == 0) s_carry = SEEDED ? seed_in[f] : ring[(int64_t)f * cap + start];
   __syncthreads();
   const int n_main = nw - 1;                 // windows with the full decay; the last window is folded in afterwards
   for (int row = 0; row * 128 < n_main; ++row) {
@@ -997,7 +1001,11 @@ __global__ void __launch_bounds__(128) k_ema_carry(const double* __restrict__ pa
     if (w == min(n_main, (row + 1) * 128) - 1) s_carry = e;   // the row's last valid window carries into the next row
     __syncthreads();
   }
-  if (t == 0) O[nw - 1] = fma(d_last, s_carry, __ldg(P + nw - 1));
+  if (t == 0) {
+    const double e = fma(d_last, s_carry, __ldg(P + nw - 1));
+    O[nw - 1] = e;
+    if (seed_out) seed_out[f] = e;
+  }
 }
 
 }  // namespace
@@ -1050,6 +1058,18 @@ struct gpud_ring {
   int range_reasons[GPUD_RANGE_N_OPEN_REASONS] = {0};
   int range_fields_open = 0;                           // fields the last sampled reduce_range handed to the histogram path
   cudaEvent_t ev_k[3] = {nullptr, nullptr, nullptr};   // around the two kernels of the last reduce (bench roofline)
+  // streaming drain (gpud_ring_drain): its own scratch, so a drain never changes what gpud_ring_read returns
+  int64_t drain_next = 0;                              // first stream window not drained yet
+  int64_t ema_window = -1;                             // the window whose EMA d_ema_state holds (-1: none)
+  int64_t export_last_ms = INT64_MIN;                  // time the store writer gave the newest window it exported
+  int64_t last_timed_ms = INT64_MIN;                   // time of the newest row that came through gpud_ring_push_timed
+  std::vector<int64_t> win_ms;                         // [nw_max + 2]: end time of window k at k % size (0 = untimed)
+  int64_t dr_chunk = 0;                                // windows per drain launch (the scratch below holds [F][dr_chunk])
+  double* d_dr[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // min, max, mean, ema, p99
+  uint32_t* d_dr_nover = nullptr;
+  double* d_dr_part = nullptr;                         // per-window EMA partials
+  double* d_ema_state = nullptr;                       // [F] EMA of window ema_window (committed)
+  double* d_ema_pend = nullptr;                        // [F] EMA of the last window of the current peek
 };
 
 static int64_t ring_count(const gpud_ring* r) { return std::min(r->total, r->cap); }
@@ -1074,6 +1094,7 @@ extern "C" int32_t gpud_ring_create(gpud_ctx* ctx, int32_t dev, const gpud_ring_
   { const char* env = getenv("GPUD_WINDOW_LANDING"); r->tma_landing = env && !strcmp(env, "tma"); r->inplace_landing = env && !strcmp(env, "inplace"); }
 #endif
   r->nw_max = (r->cap + r->W - 1) / r->W;
+  r->win_ms.assign((size_t)r->nw_max + 2, 0);
   const size_t ring_bytes = (size_t)r->F * r->cap * sizeof(double) + 64;   // slack: the 16-byte load of a window's last odd element
   const size_t res_bytes = (size_t)r->F * r->nw_max * sizeof(double);
   while (((r->cap + (1ll << r->smp_shift) - 1) >> r->smp_shift) > GPUD_RANGE_SAMPLE_MAX) ++r->smp_shift;
@@ -1129,6 +1150,8 @@ extern "C" int32_t gpud_ring_destroy(gpud_ring* r) {
   cudaFree(r->d_rng_nover);
   cudaFree(r->d_rng_cls); cudaFree(r->d_rng_lists); cudaFree(r->d_rng_piv);
   for (auto& ev : r->ev_rng) if (ev) cudaEventDestroy(ev);
+  for (auto& p : r->d_dr) cudaFree(p);
+  cudaFree(r->d_dr_nover); cudaFree(r->d_dr_part); cudaFree(r->d_ema_state); cudaFree(r->d_ema_pend);
   for (int i = 0; i < 2; ++i) {
     if (r->h_stage[i]) cudaFreeHost(r->h_stage[i]);
     cudaFree(r->d_stage[i]);
@@ -1192,17 +1215,53 @@ static int32_t launch_append(gpud_ring* r, const void* d_rows, int64_t n, int32_
   return GPUD_OK;
 }
 
+// Record the end time of every window the rows [old_total, total) completed: row_ms[i] is the time of row old_total + i, NULL = untimed
+// (0).  Only the newest win_ms.size() windows can still be drained (the ring holds at most nw_max of them), so older ones are skipped.
+static void stamp_windows(gpud_ring* r, int64_t old_total, const int64_t* row_ms) {
+  const int64_t sz = (int64_t)r->win_ms.size();
+  const int64_t k_end = r->total / r->W;
+  const int64_t k_begin = std::max(old_total / r->W, k_end - sz);
+  for (int64_t k = k_begin; k < k_end; ++k) r->win_ms[k % sz] = row_ms ? row_ms[(k + 1) * r->W - 1 - old_total] : 0;
+}
+
 extern "C" int32_t gpud_ring_push_device(gpud_ring* r, const double* dev_rows, int64_t n) {
   if (!r || (!dev_rows && n) || n < 0) return GPUD_E_INVALID;
   if (n == 0) return GPUD_OK;
   GPUD_CUDA(r->ctx, cudaSetDevice(r->dev));
-  return launch_append(r, dev_rows, n, GPUD_DT_F64);
+  const int64_t old_total = r->total;
+  const int32_t rc = launch_append(r, dev_rows, n, GPUD_DT_F64);
+  stamp_windows(r, old_total, nullptr);
+  return rc;
 }
 
+static int32_t push_host(gpud_ring* r, const void* host_rows_v, int64_t n, int32_t dt);
+
 extern "C" int32_t gpud_ring_push_raw(gpud_ring* r, const void* host_rows_v, int64_t n, int32_t dt) {
-  const size_t esz = dtype_size(dt);
-  if (!r || (!host_rows_v && n) || n < 0 || esz == 0) return GPUD_E_INVALID;
+  if (!r || (!host_rows_v && n) || n < 0 || dtype_size(dt) == 0) return GPUD_E_INVALID;
   if (n == 0) return GPUD_OK;
+  const int64_t old_total = r->total;
+  const int32_t rc = push_host(r, host_rows_v, n, dt);
+  stamp_windows(r, old_total, nullptr);
+  return rc;
+}
+
+extern "C" int32_t gpud_ring_push_timed(gpud_ring* r, const void* host_rows_v, int64_t n, int32_t dt, const int64_t* row_ms) {
+  if (!r || (!host_rows_v && n) || (!row_ms && n) || n < 0 || dtype_size(dt) == 0) return GPUD_E_INVALID;
+  if (n == 0) return GPUD_OK;
+  if (row_ms[0] < r->last_timed_ms)
+    return gpud_fail(r->ctx, GPUD_E_INVALID, "push_timed: row time %lld is earlier than the last timed row (%lld)", (long long)row_ms[0], (long long)r->last_timed_ms);
+  for (int64_t i = 1; i < n; ++i)
+    if (row_ms[i] < row_ms[i - 1]) return gpud_fail(r->ctx, GPUD_E_INVALID, "push_timed: row times decrease at row %lld", (long long)i);
+  const int64_t old_total = r->total;
+  const int32_t rc = push_host(r, host_rows_v, n, dt);
+  if (r->total > old_total) r->last_timed_ms = row_ms[r->total - old_total - 1];
+  stamp_windows(r, old_total, row_ms);
+  return rc;
+}
+
+// the body of gpud_ring_push_raw (arguments checked, n > 0)
+static int32_t push_host(gpud_ring* r, const void* host_rows_v, int64_t n, int32_t dt) {
+  const size_t esz = dtype_size(dt);
   const char* host_rows = (const char*)host_rows_v;
   GPUD_CUDA(r->ctx, cudaSetDevice(r->dev));
   if (n > r->cap) {                      // rows that would be overwritten immediately never cross PCIe
@@ -1353,9 +1412,9 @@ extern "C" int32_t gpud_ring_reduce(gpud_ring* r) {
   { int32_t rc = launch_windows<false>(r, p); if (rc) return rc; }
   cudaEventRecord(r->ev_k[1], r->stream);
   const int m_last = (int)(count - (int64_t)(p.nw - 1) * r->W);
-  k_ema_carry<<<r->F, 128, 0, r->stream>>>(r->d_part, r->d_ring, r->cap, p.start, r->F, p.nw,
+  k_ema_carry<false><<<r->F, 128, 0, r->stream>>>(r->d_part, r->d_ring, r->cap, p.start, r->F, p.nw,
                                                         pow(1.0 - r->alpha, (double)r->W), pow(1.0 - r->alpha, (double)m_last),
-                                                        r->d_res[GPUD_OP_EMA]);
+                                                        r->d_res[GPUD_OP_EMA], nullptr, nullptr);
   GPUD_CUDA(r->ctx, cudaGetLastError());
   cudaEventRecord(r->ev_k[2], r->stream);
   r->reduced_nw = p.nw;
@@ -1396,6 +1455,96 @@ extern "C" int32_t gpud_ring_read(gpud_ring* r, int32_t op, void* out, int64_t o
   const void* src = op == GPUD_OP_NOVER ? (const void*)r->d_nover : (const void*)r->d_res[op];
   GPUD_CUDA(r->ctx, cudaMemcpyAsync(out, src, need, cudaMemcpyDeviceToHost, r->stream));
   GPUD_CUDA(r->ctx, cudaStreamSynchronize(r->stream));
+  return GPUD_OK;
+}
+
+// ---- streaming drain: stream-aligned windows, each reduced once, into the drain's own scratch ----
+// A drain launches the same window kernel over windows [k0, k0 + n) of the stream: physical start (k0 W) mod CAP, n W samples.  Once the
+// ring has wrapped, a window can straddle column CAP-1 -> 0 (CAP mod W != 0) or start on an odd column (odd W); launch_windows sends
+// those to the generic instantiation exactly as it does for gpud_ring_reduce.
+constexpr int64_t kDrainUnits = 1 << 20;   // (field, window) pairs per drain launch: bounds the scratch at F x chunk x 52 B
+
+static void drain_counts(const gpud_ring* r, int64_t max_windows, gpud_drain_info* info) {
+  const int64_t W = r->W, count = ring_count(r);
+  const int64_t complete = r->total / W;
+  const int64_t k0 = std::max(r->drain_next, (r->total - count + W - 1) / W);
+  const int64_t avail = complete - k0;
+  info->first_window = k0;
+  info->n_windows = std::min(avail, max_windows);
+  info->n_lost = k0 - r->drain_next;
+  info->n_pending = avail - info->n_windows;
+}
+
+int32_t gpud_ring_drain_peek(gpud_ring* r, int64_t max_windows, double* out_f64, uint32_t* out_nover, int64_t* out_ms, gpud_drain_info* info) {
+  drain_counts(r, max_windows, info);
+  const int64_t k0 = info->first_window, n = info->n_windows;
+  if (n == 0) return GPUD_OK;
+  GPUD_CUDA(r->ctx, cudaSetDevice(r->dev));
+  if (!r->d_ema_state) {
+    for (auto& p : r->d_dr) { cudaFree(p); p = nullptr; }      // whatever an earlier, failed attempt left
+    cudaFree(r->d_dr_nover); cudaFree(r->d_dr_part); cudaFree(r->d_ema_pend);
+    r->d_dr_nover = nullptr; r->d_dr_part = r->d_ema_pend = nullptr;
+    r->dr_chunk = std::max<int64_t>(1, std::min<int64_t>(r->nw_max, kDrainUnits / r->F));
+    const size_t per = (size_t)r->F * r->dr_chunk;
+    for (int i = 0; i < 5; ++i) GPUD_CUDA(r->ctx, cudaMalloc(&r->d_dr[i], per * sizeof(double)));
+    GPUD_CUDA(r->ctx, cudaMalloc(&r->d_dr_nover, per * sizeof(uint32_t)));
+    GPUD_CUDA(r->ctx, cudaMalloc(&r->d_dr_part, per * sizeof(double)));
+    GPUD_CUDA(r->ctx, cudaMalloc(&r->d_ema_pend, r->F * sizeof(double)));
+    GPUD_CUDA(r->ctx, cudaMalloc(&r->d_ema_state, r->F * sizeof(double)));   // allocated last: its presence means the scratch is complete
+  }
+  // the EMA continues from the previous drain only when that drain ended on window k0 - 1 (no loss in between)
+  const bool carry = k0 > 0 && r->ema_window == k0 - 1;
+  const double d_w = pow(1.0 - r->alpha, (double)r->W);
+  for (int64_t j0 = 0; j0 < n; j0 += r->dr_chunk) {
+    const int64_t nc = std::min(r->dr_chunk, n - j0);
+    WinParams p;
+    p.ring = r->d_ring; p.cap = r->cap; p.start = ((k0 + j0) * r->W) % r->cap; p.count = nc * r->W;
+    p.W = r->W; p.F = r->F; p.nw = (int)nc;
+    p.q_num = r->q_num; p.q_den = r->q_den; p.thr = r->d_thr; p.pw = r->d_pw; p.pwl = r->d_pwl;
+    p.q64 = pow(1.0 - r->alpha, 64.0); p.alpha = r->alpha;
+    p.out_min = r->d_dr[GPUD_OP_MIN]; p.out_max = r->d_dr[GPUD_OP_MAX]; p.out_mean = r->d_dr[GPUD_OP_MEAN];
+    p.out_p99 = r->d_dr[GPUD_OP_P99]; p.out_nover = r->d_dr_nover; p.part = r->d_dr_part; p.do_select = 1;
+    { int32_t rc = launch_windows<false>(r, p); if (rc) return rc; }
+    if (j0 == 0 && !carry)
+      k_ema_carry<false><<<r->F, 128, 0, r->stream>>>(r->d_dr_part, r->d_ring, r->cap, p.start, r->F, (int)nc, d_w, d_w, r->d_dr[GPUD_OP_EMA],
+                                                       nullptr, r->d_ema_pend);
+    else
+      k_ema_carry<true><<<r->F, 128, 0, r->stream>>>(r->d_dr_part, r->d_ring, r->cap, p.start, r->F, (int)nc, d_w, d_w, r->d_dr[GPUD_OP_EMA],
+                                                      j0 == 0 ? r->d_ema_state : r->d_ema_pend, r->d_ema_pend);
+    GPUD_CUDA(r->ctx, cudaGetLastError());
+    // only the nc new windows cross PCIe, one strided copy per output straight into the caller's layout
+    for (int op = 0; op < 5; ++op)
+      GPUD_CUDA(r->ctx, cudaMemcpy2DAsync(out_f64 + ((size_t)op * r->F) * max_windows + j0, (size_t)max_windows * sizeof(double), r->d_dr[op],
+                                          (size_t)nc * sizeof(double), (size_t)nc * sizeof(double), (size_t)r->F, cudaMemcpyDeviceToHost, r->stream));
+    GPUD_CUDA(r->ctx, cudaMemcpy2DAsync(out_nover + j0, (size_t)max_windows * sizeof(uint32_t), r->d_dr_nover, (size_t)nc * sizeof(uint32_t),
+                                        (size_t)nc * sizeof(uint32_t), (size_t)r->F, cudaMemcpyDeviceToHost, r->stream));
+  }
+  GPUD_CUDA(r->ctx, cudaStreamSynchronize(r->stream));
+  if (out_ms) {
+    const int64_t sz = (int64_t)r->win_ms.size();
+    for (int64_t j = 0; j < n; ++j) out_ms[j] = r->win_ms[(k0 + j) % sz];
+  }
+  return GPUD_OK;
+}
+
+void gpud_ring_drain_commit(gpud_ring* r, const gpud_drain_info* info, int64_t last_export_ms) {
+  r->drain_next = info->first_window + info->n_windows;
+  if (info->n_windows > 0) {
+    // stream-ordered after the peek's carry kernel; both buffers are only ever read by later launches on the same stream
+    cudaSetDevice(r->dev);
+    cudaMemcpyAsync(r->d_ema_state, r->d_ema_pend, r->F * sizeof(double), cudaMemcpyDeviceToDevice, r->stream);
+    r->ema_window = r->drain_next - 1;
+  }
+  if (last_export_ms != INT64_MIN) r->export_last_ms = last_export_ms;
+}
+
+int64_t gpud_ring_drain_last_export(const gpud_ring* r) { return r->export_last_ms; }
+
+extern "C" int32_t gpud_ring_drain(gpud_ring* r, int64_t max_windows, double* out_f64, uint32_t* out_nover, int64_t* out_ms, gpud_drain_info* info) {
+  if (!r || !info || max_windows < 0 || (max_windows > 0 && (!out_f64 || !out_nover))) return GPUD_E_INVALID;
+  const int32_t rc = gpud_ring_drain_peek(r, max_windows, out_f64, out_nover, out_ms, info);
+  if (rc) return rc;
+  if (max_windows > 0) gpud_ring_drain_commit(r, info, INT64_MIN);
   return GPUD_OK;
 }
 
@@ -1456,8 +1605,8 @@ int32_t gpud_ring_range_pass(gpud_ring* r, const gpud_range_view* v) {
   p.piv = v->piv; p.w_cls = v->w_cls; p.lists = v->lists; p.fill = v->fill; p.list_cap = v->list_cap;
   { int32_t rc = v->sampled ? launch_windows<true>(r, p) : launch_windows<false>(r, p); if (rc) return rc; }
   const int m_last = (int)(v->n - (int64_t)(v->nw - 1) * v->Wp);
-  k_ema_carry<<<r->F, 128, 0, r->stream>>>(r->d_rng[4], r->d_ring, r->cap, v->start, r->F, v->nw, pow(1.0 - r->alpha, (double)v->Wp),
-                                                        pow(1.0 - r->alpha, (double)m_last), r->d_rng[3]);
+  k_ema_carry<false><<<r->F, 128, 0, r->stream>>>(r->d_rng[4], r->d_ring, r->cap, v->start, r->F, v->nw, pow(1.0 - r->alpha, (double)v->Wp),
+                                                        pow(1.0 - r->alpha, (double)m_last), r->d_rng[3], nullptr, nullptr);
   GPUD_CUDA(r->ctx, cudaGetLastError());
   return GPUD_OK;
 }

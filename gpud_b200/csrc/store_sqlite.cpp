@@ -3,7 +3,8 @@
 //   events   pkg/eventstore/database.go:18-31 (schema version, columns), :136-143 (table name), :198-246 (createTable),
 //            :248-275 (insertEvent: NULLIF(?, '') for message / extra_info), :277-324 (findEvent duplicate check)
 //   metrics  pkg/metrics/store/sqlite.go:22-36 (schema version, columns, default table), :87-106 (CreateTable),
-//            :108-164 (insert: INSERT OR REPLACE, labels as JSON or '')
+//            :108-164 (insert: INSERT OR REPLACE, labels as JSON or ''), :258-275 (purge)
+//   window rows  what the Syncer (pkg/metrics/syncer/syncer.go:76-82) records on its ticker, from the ring's streaming drain
 //   xid events as persisted by xid/component.go:503-554 (name "error_xid", extra_info {"data", "device_uuid"})
 // SQLite itself is dlopen'ed (libsqlite3.so.0; the image carries the library but no headers), WAL + busy timeout like
 // pkg/sqlite (SURVEY.md §2: `_journal_mode=WAL&_busy_timeout=5000`).
@@ -13,12 +14,14 @@
 #include <string.h>
 #include <time.h>
 
+#include <algorithm>
 #include <map>
 #include <string>
 #include <vector>
 
 #include "../../include/gpud_b200.h"
 #include "json_min.h"
+#include "ring_drain.h"
 
 namespace {
 
@@ -607,6 +610,118 @@ extern "C" int32_t gpud_store_record_metrics(gpud_store* st, const char* table, 
   }
   S->finalize(q);
   if (S->exec(st->db, "COMMIT;", nullptr, nullptr, nullptr) != kOk) return sfail(st, "commit");
+  return GPUD_OK;
+}
+
+// metrics/store/sqlite.go:258-275 (purge)
+extern "C" int32_t gpud_store_purge_metrics(gpud_store* st, const char* table, int64_t before_unix_ms, int64_t* n_purged) {
+  if (!st) return GPUD_E_INVALID;
+  Sq* S = sq();
+  if (!S) return GPUD_E_UNSUPPORTED;
+  const std::string t = table && *table ? table : "gpud_metrics_v0_5";
+  if (!ident_ok(t.c_str())) return GPUD_E_INVALID;
+  const std::string del = "\nDELETE FROM " + t + " WHERE unix_milliseconds < ?;";
+  void* q = nullptr;
+  if (S->prepare_v2(st->db, del.c_str(), -1, &q, nullptr) != kOk) return sfail(st, "prepare metrics purge");
+  S->bind_int64(q, 1, before_unix_ms);
+  const int rc = S->step(q);
+  S->finalize(q);
+  if (rc != kDone) return sfail(st, "purge metrics");
+  if (n_purged) *n_purged = S->changes(st->db);
+  return GPUD_OK;
+}
+
+extern "C" int32_t gpud_window_metric_name(const char* field, int32_t op, int32_t q_num, int32_t q_den, char* out, int32_t cap) {
+  if (!field || !out || op < 0 || op >= GPUD_N_OPS || q_num < 0 || q_den <= 0 || q_num > q_den) return -1;
+  static const char* const kOp[GPUD_N_OPS] = {"min", "max", "mean", "ema", nullptr, "n_over"};
+  char q[64];
+  const char* suffix = kOp[op];
+  if (op == GPUD_OP_P99) {
+    char g[48];
+    snprintf(g, sizeof g, "%g", 100.0 * q_num / q_den);
+    for (char* c = g; *c; ++c) if (*c == '.') *c = '_';
+    snprintf(q, sizeof q, "p%s", g);
+    suffix = q;
+  }
+  const std::string name = std::string(field) + "_window_" + suffix;
+  if ((int32_t)name.size() + 1 > cap) return -1;
+  memcpy(out, name.c_str(), name.size() + 1);
+  return (int32_t)name.size();
+}
+
+// Syncer.sync (syncer.go:76-82) over a ring: peek the next windows, write them in one transaction, and only then move the ring's cursor
+extern "C" int32_t gpud_ring_drain_to_store(gpud_ring* ring, gpud_store* st, const char* table, const char* const* components, const char* const* field_names,
+                                            const char* labels_json, uint32_t ops_mask, int64_t max_windows, gpud_drain_info* info, int64_t* n_rows,
+                                            int64_t* n_shifted) {
+  if (!ring || !st || !components || !field_names || max_windows < 0 || ops_mask >= (1u << GPUD_N_OPS)) return GPUD_E_INVALID;
+  Sq* S = sq();
+  if (!S) return GPUD_E_UNSUPPORTED;
+  const std::string t = table && *table ? table : "gpud_metrics_v0_5";
+  if (!ident_ok(t.c_str())) return GPUD_E_INVALID;
+  const int F = gpud_ring_n_fields(ring);
+  for (int f = 0; f < F; ++f)
+    if (field_names[f] && (!*field_names[f] || !components[f] || !*components[f])) return GPUD_E_INVALID;   // ErrEmptyComponentName / ErrEmptyMetricName
+  if (ops_mask == 0) ops_mask = (1u << GPUD_N_OPS) - 1;
+  gpud_drain_info di;
+  if (n_rows) *n_rows = 0;
+  if (n_shifted) *n_shifted = 0;
+  // counts first, so that the host arrays hold the windows that come back rather than max_windows of them
+  int32_t rc = gpud_ring_drain_peek(ring, 0, nullptr, nullptr, nullptr, &di);
+  const int64_t want = std::min(max_windows, di.n_pending);
+  const size_t mw = (size_t)want;
+  std::vector<double> f64(5 * (size_t)F * mw + 1);
+  std::vector<uint32_t> nov((size_t)F * mw + 1);
+  std::vector<int64_t> ms(mw + 1);
+  if (rc == GPUD_OK && want > 0) rc = gpud_ring_drain_peek(ring, want, f64.data(), nov.data(), ms.data(), &di);
+  if (rc) { st->err = "drain: the ring's reduce failed (see gpud_last_error)"; return rc; }
+  if (info) *info = di;
+  if (max_windows == 0) return GPUD_OK;                                         // a query
+  const int64_t n = di.n_windows;
+  for (int64_t j = 0; j < n; ++j)
+    if (ms[j] == 0) {
+      st->err = "window " + std::to_string(di.first_window + j) + " has no time (its last row was pushed without one)";
+      return GPUD_E_STATE;
+    }
+  // unix_milliseconds leads the primary key: a window that does not come after the previous exported one moves to 1 ms after it
+  int64_t prev = gpud_ring_drain_last_export(ring), shifted = 0;
+  for (int64_t j = 0; j < n; ++j) {
+    if (prev != INT64_MIN && ms[j] <= prev) { ms[j] = prev + 1; ++shifted; }
+    prev = ms[j];
+  }
+  int qn = 99, qd = 100;
+  gpud_ring_quantile(ring, &qn, &qd);
+  std::vector<std::string> names((size_t)F * GPUD_N_OPS);
+  for (int f = 0; f < F; ++f)
+    for (int op = 0; op < GPUD_N_OPS; ++op)
+      if (field_names[f] && ((ops_mask >> op) & 1u)) {
+        char b[512];
+        if (gpud_window_metric_name(field_names[f], op, qn, qd, b, sizeof b) < 0) return GPUD_E_INVALID;
+        names[(size_t)f * GPUD_N_OPS + op] = b;
+      }
+  int64_t rows = 0;
+  if (n > 0) {
+    const std::string ins = "INSERT OR REPLACE INTO " + t + " (unix_milliseconds, component_name, metric_name, metric_labels, metric_value) VALUES (?, ?, ?, ?, ?)";
+    void* q = nullptr;
+    if (S->exec(st->db, "BEGIN;", nullptr, nullptr, nullptr) != kOk) return sfail(st, "begin");
+    if (S->prepare_v2(st->db, ins.c_str(), -1, &q, nullptr) != kOk) { rc = sfail(st, "prepare metrics insert"); S->exec(st->db, "ROLLBACK;", nullptr, nullptr, nullptr); return rc; }
+    for (int64_t j = 0; j < n; ++j)
+      for (int f = 0; f < F; ++f)
+        for (int op = 0; op < GPUD_N_OPS; ++op) {
+          const std::string& name = names[(size_t)f * GPUD_N_OPS + op];
+          if (name.empty()) continue;
+          const double v = op == GPUD_OP_NOVER ? (double)nov[(size_t)f * mw + j] : f64[((size_t)op * F + f) * mw + j];
+          S->bind_int64(q, 1, ms[j]); S->bind_text(q, 2, components[f], -1, kTransient); S->bind_text(q, 3, name.c_str(), -1, kTransient);
+          S->bind_text(q, 4, labels_json ? labels_json : "", -1, kTransient); S->bind_double(q, 5, v);
+          if (S->step(q) != kDone) { rc = sfail(st, "insert metric"); S->finalize(q); S->exec(st->db, "ROLLBACK;", nullptr, nullptr, nullptr); return rc; }
+          S->reset(q);
+          ++rows;
+        }
+    S->finalize(q);
+    if (S->exec(st->db, "COMMIT;", nullptr, nullptr, nullptr) != kOk) { rc = sfail(st, "commit"); S->exec(st->db, "ROLLBACK;", nullptr, nullptr, nullptr); return rc; }
+  }
+  gpud_ring_drain_commit(ring, &di, n > 0 ? prev : INT64_MIN);
+  if (n_rows) *n_rows = rows;
+  if (n_shifted) *n_shifted = shifted;
   return GPUD_OK;
 }
 

@@ -39,7 +39,8 @@ typedef struct gpud_ring gpud_ring;
 int32_t gpud_abi_version(void);
 /* sizeof of the ABI structs for binding layout checks (5 gpud_kmsg_event, 6 gpud_ib_snapshot, 7 gpud_ib_verdict, 8 gpud_metric):
  * 0 gpud_xid_hit, 1 gpud_fabric_raw, 2 gpud_fabric_local,
- * 3 gpud_fabric_verdict, 4 gpud_ring_cfg, 9 gpud_dedup_rule .. 12 gpud_event_row, 13 gpud_nvml_device, 14 gpud_remapped_rows, 15 gpud_ecc_errors, 16 gpud_gpm_metrics; -1 otherwise. */
+ * 3 gpud_fabric_verdict, 4 gpud_ring_cfg, 9 gpud_dedup_rule .. 12 gpud_event_row, 13 gpud_nvml_device, 14 gpud_remapped_rows, 15 gpud_ecc_errors, 16 gpud_gpm_metrics,
+ * 17 gpud_drain_info; -1 otherwise. */
 int32_t gpud_sizeof(int32_t which);
 
 /* One context per process; `cuda_devs[n]` are the CUDA ordinals this process drives (one per rank when
@@ -109,8 +110,9 @@ int32_t gpud_hw_slowdown_check(const int64_t* event_unix, int32_t n, int64_t now
 /* Real ingest (SURVEY.md 8f.3): a host poller that reads the NVML gauges of CUDA device `dev` - the getters behind the
  * reference's temperature / power / clock-speed / utilization / memory components (temperature/temperature.go:85,
  * power/power.go:46, clock-speed/clock_speed.go:41,59, utilization/utilization.go:44, memory/memory.go:83) - into pinned
- * uint32 poll rows and appends them to `ring` with gpud_ring_push_raw.  The ring must have GPUD_POLL_N_FIELDS fields, in this
- * column order.  NVML is dlopen'ed; GPUD_E_UNSUPPORTED if the host has no driver library. */
+ * uint32 poll rows and appends them to `ring` with gpud_ring_push_timed.  The ring must have GPUD_POLL_N_FIELDS fields, in this
+ * column order.  NVML is dlopen'ed; GPUD_E_UNSUPPORTED if the host has no driver library.  Every row is pushed with the wall-clock ms its
+ * getters returned at (gpud_ring_push_timed), as are the rows of gpud_poller_poll_fields and gpud_poller_poll_gpm. */
 enum { GPUD_POLL_TEMPERATURE_C = 0, GPUD_POLL_POWER_MW = 1, GPUD_POLL_CLOCK_GRAPHICS_MHZ = 2, GPUD_POLL_CLOCK_SM_MHZ = 3,
        GPUD_POLL_CLOCK_MEM_MHZ = 4, GPUD_POLL_UTIL_GPU_PCT = 5, GPUD_POLL_UTIL_MEM_PCT = 6, GPUD_POLL_MEMORY_USED_MIB = 7,
        GPUD_POLL_N_FIELDS = 8 };
@@ -235,6 +237,25 @@ enum { GPUD_RANGE_OPEN_SHORT = 1,    /* the range is shorter than the single-pas
        GPUD_RANGE_OPEN_OVERFLOW = 6, /* more keys between the pivots than the list holds              */
        GPUD_RANGE_N_OPEN_REASONS = 7 };
 int32_t gpud_ring_range_stats(gpud_ring* ring, float* pass_ms, float* total_ms, int32_t* fields_by_histogram, int32_t* reasons);
+
+/* Streaming windows: what a metrics syncer (pkg/metrics/syncer/syncer.go:76-82, which scrapes the gauges of
+ * pkg/metrics/scraper/prometheus.go:28-81 on its ticker) reads from the ring instead of the gauges.  Sample i of a field is the i-th
+ * sample pushed since gpud_ring_create (rows a push skips because n_rows > CAP still count); window k is samples [kW, (k+1)W), complete
+ * once (k+1)W <= total.  The ring keeps a cursor `next` (first window not drained yet, initially 0).  A drain returns complete windows
+ * from k0 = max(next, ceil((total - count) / W)) upward, oldest first, each reduced on the GPU exactly once:
+ *   n_lost = k0 - next windows were overwritten before they were drained; n_windows = min(floor(total / W) - k0, max_windows) are
+ *   returned (window first_window + j); n_pending complete windows remain.  Afterwards next = k0 + n_windows.  max_windows = 0 is a
+ *   query: *info is filled and nothing moves.
+ * min / max / p<q> / n_over / mean are the aggregates of gpud_ring_reduce over the window's W samples.  The EMA runs over the stream and
+ * continues from the last window the previous drain returned, except on the first drain and after a loss, where it starts at the first
+ * sample of the first returned window.  Output: out_f64[(op * F + f) * max_windows + j] for op GPUD_OP_MIN .. GPUD_OP_P99,
+ * n_over[f * max_windows + j], window_end_unix_ms[j] (may be NULL) = the time of the window's last row when that row came through
+ * gpud_ring_push_timed, else 0.  The results of gpud_ring_reduce / gpud_ring_read are not touched.  Synchronous. */
+typedef struct { int64_t first_window, n_windows, n_lost, n_pending; } gpud_drain_info;
+int32_t gpud_ring_drain(gpud_ring* ring, int64_t max_windows, double* out_f64, uint32_t* out_n_over, int64_t* window_end_unix_ms, gpud_drain_info* info);
+/* gpud_ring_push_raw with the time each row was read (unix ms, row_unix_ms[n_rows]): non-decreasing within the call and not earlier
+ * than the last timed row, else GPUD_E_INVALID and nothing is appended.  Untimed pushes give the windows they complete time 0. */
+int32_t gpud_ring_push_timed(gpud_ring* ring, const void* host_rows, int64_t n_rows, int32_t dtype, const int64_t* row_unix_ms);
 
 /* ------------------------------------------------------------------------------------------------
  * components.Component (components/types.go:20-66) for the three paths this library replaces, as objects: what a Go file that
@@ -526,6 +547,28 @@ int32_t gpud_kmsg_syncer_feed(gpud_kmsg_syncer* sy, const char* kmsg_component, 
 /* table NULL or "" = "gpud_metrics_v0_5" (metrics/store/sqlite.go:36) */
 int32_t gpud_store_metrics_table(gpud_store* st, const char* table);
 int32_t gpud_store_record_metrics(gpud_store* st, const char* table, const gpud_metric* ms, int64_t n);
+/* purge (metrics/store/sqlite.go:258-275): DELETE the rows with unix_milliseconds < before_unix_ms; the reference Syncer runs it on its
+ * own ticker (syncer.go:55-71) so that a table fed every tick does not grow without bound. */
+int32_t gpud_store_purge_metrics(gpud_store* st, const char* table, int64_t before_unix_ms, int64_t* n_purged);
+/* Name of a drained window aggregate: "<field>_window_<op>", op = min | max | mean | ema | p<Q> | n_over (GPUD_OP_*), Q = printf("%g",
+ * 100 q_num / q_den) with '.' -> '_' (99/100 -> p99, 999/1000 -> p99_9: Prometheus names have no '.').  Returns the length, -1 if cap
+ * is too small. */
+int32_t gpud_window_metric_name(const char* field, int32_t op, int32_t q_num, int32_t q_den, char* out, int32_t cap);
+/* The Syncer's sync step (syncer.go:76-82) over a ring: gpud_ring_drain, then one metrics row (store/sqlite.go:108-164, INSERT OR
+ * REPLACE) per returned window x field whose field_names[f] is not NULL x op of ops_mask (bit GPUD_OP_*; 0 = all six):
+ * component_name components[f], metric_name gpud_window_metric_name(field_names[f], ...), metric_labels labels_json (rendered like
+ * json.Marshal: sorted keys, no spaces; "" = none), metric_value (n_over as REAL), unix_milliseconds the window's end time.  A window
+ * without a time fails the call with GPUD_E_STATE.  A window whose time is not after the previous exported window of this ring is
+ * written 1 ms after it (counted in *n_shifted), so that two windows never share a primary key.  Atomic: all rows in one transaction,
+ * and the ring's cursor and EMA state advance only after COMMIT; on any failure the store, the cursor and the EMA are as they were and
+ * the next call returns the same windows.  *n_rows = rows written. */
+int32_t gpud_ring_drain_to_store(gpud_ring* ring, gpud_store* st, const char* table, const char* const* components, const char* const* field_names,
+                                 const char* labels_json, uint32_t ops_mask, int64_t max_windows, gpud_drain_info* info, int64_t* n_rows, int64_t* n_shifted);
+/* temperature component only: while a store is attached (st = NULL detaches), every Check drains each GPU's ring into `table` right
+ * after the poll, with all six ops, labels {"uuid":"<uuid>"} and the reference gauges' names (INTEGRATION.md).  A failed drain leaves
+ * the Check result alone, as the reference Syncer only logs; the message goes to gpud_last_error and the windows stay for the next
+ * tick.  GPUD_E_INVALID for other components. */
+int32_t gpud_component_set_metrics_store(gpud_component* c, gpud_store* st, const char* table);
 
 /* InfiniBand port drop / flap scans (SURVEY.md 8f.4): findDrops / findFlaps of
  * components/accelerator/nvidia/infiniband/store/scan_drops.go:41-116 and scan_flaps.go:47-134 over many (device, port)
